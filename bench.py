@@ -71,7 +71,26 @@ def parse_args():
                     help="clock samplers running during the timed regions (A/B their perturbation with 'none')")
     ap.add_argument("--replica-pick", default="balanced", choices=["balanced", "hot-spread", "random", "first", "hash"],
                     help="replica choice among the ring's GetN candidates (reference: random)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last one as DIR/predict_y.npy (float32, at most 64 MB: "
+                         "a larger result is cut to a fixed seeded sample of its rows); at N > 1 one file per rank, predict_y_rank<r>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 path only")
+    return a
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def sample_rows(y: np.ndarray, max_bytes: int, seed: int = 0) -> np.ndarray:
+    """y itself when it fits in max_bytes, else a fixed seeded sample of its rows, kept in their original order."""
+    keep = max_bytes // max(1, y[:1].nbytes)
+    if len(y) <= keep:
+        return y
+    return y[np.sort(np.random.default_rng(seed).choice(len(y), keep, replace=False))]
 
 
 def effective_cpus() -> int:
@@ -476,7 +495,8 @@ def run_b200(args):
     sptr = stream.cuda_stream
     assert sptr != 0
     max_rows = args.tick * 4
-    x_dev = torch.randn(max_rows, in_dim, device="cuda", dtype=torch.float32)
+    x_dev = torch.randn(max_rows, in_dim, device="cuda", dtype=torch.float32,
+                        generator=torch.Generator(device="cuda").manual_seed(0))   # same inputs in every run (--dump-outputs)
     y_dev = torch.empty(max_rows, out_dim, device="cuda", dtype=torch.float32)
     xb_dev = torch.empty(max_rows, in_dim, device="cuda", dtype=torch.float32)    # gathered batches (groups with forwarded rows)
     yb_dev = torch.empty(max_rows, out_dim, device="cuda", dtype=torch.float32)
@@ -511,6 +531,7 @@ def run_b200(args):
         launches, gsegs, ssegs = [], [], []
         loff = boff = 0
         fwd_rows = 0
+        fwd_idx = []   # rows of yb_dev that hold the results of forwarded requests
         for m, n_local, fl in groups:
             n = n_local + len(fl)
             if not fl:
@@ -526,13 +547,14 @@ def run_b200(args):
             for j, (p, k) in enumerate(fl):
                 gsegs.append((pwin[p] + k * inb, xb + (n_local + j) * inb, inb))                      # NVLink read
                 ssegs.append((yb + (n_local + j) * outb, pwin[p] + y_base + k * outb, outb))          # NVLink write
+                fwd_idx.append(boff + n_local + j)
             launches.append((f"m{m}".encode(), n, xb, yb))
             boff += n
             fwd_rows += len(fl)
         ga = (SegArr * len(gsegs))(*[SegArr(a, b, c) for a, b, c in gsegs]) if gsegs else None
         sa = (SegArr * len(ssegs))(*[SegArr(a, b, c) for a, b, c in ssegs]) if ssegs else None
         plans[s] = dict(groups=[(m, nl + len(fl)) for m, nl, fl in groups], launches=launches, gather=ga, n_g=len(gsegs),
-                        scatter=sa, n_s=len(ssegs), fwd_rows=fwd_rows)
+                        scatter=sa, n_s=len(ssegs), fwd_rows=fwd_rows, n_local=loff, fwd_idx=fwd_idx)
     lib = _lib.lib
     h = srv._h
 
@@ -591,6 +613,14 @@ def run_b200(args):
     my_elapsed_ms, my_req = elapsed_ms, n_req
     launches = lib.tfsc_kernel_launches() - launches0
     st1 = srv.stats()
+    if args.dump_outputs:
+        # the results of the last timed step as its callers receive them: the rows of the requests that entered here, then
+        # those computed here for requests that entered at another rank (each request once over all ranks), in plan order
+        last = plans[W + K - 1]
+        y = torch.cat([y_dev[:last["n_local"]], yb_dev[torch.tensor(last["fwd_idx"], dtype=torch.long, device="cuda")]])
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "predict_y.npy" if world == 1 else f"predict_y_rank{rank}.npy"),
+                sample_rows(y.cpu().numpy(), DUMP_MAX_BYTES // world))
 
     _phase(rank, t_start, "value region done")
     # ---- e2e: host buffers through the C ABI, closed-loop clients ----------------------------------------------

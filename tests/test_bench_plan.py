@@ -4,6 +4,7 @@ import os
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -41,3 +42,17 @@ def test_single_gpu_has_no_forwarding():
     wl = bench.build_workload(1, 8, 64, 2, forward_frac=0.25)
     assert np.array_equal(wl["ingress"], wl["dest"]) and wl["forward_frac"] == 0.0
     assert all(not fl for _m, _n, fl in bench.step_plan(wl, 0, 0, 64))
+
+
+def test_dumped_sample_is_fixed_ordered_and_bounded():
+    y = np.arange(1000 * 16, dtype=np.float32).reshape(1000, 16)
+    assert bench.sample_rows(y, y.nbytes) is y
+    s = bench.sample_rows(y, 100 * y[0].nbytes + 7)
+    assert s.shape == (100, 16) and np.array_equal(s, bench.sample_rows(y, 100 * y[0].nbytes + 7))
+    assert np.all(np.diff(s[:, 0]) > 0) and np.all(s[:, 0] % 16 == 0)   # whole rows, in their original order
+
+
+def test_bench_rejects_runs_without_timed_steps(monkeypatch):
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse_args()
